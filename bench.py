@@ -23,6 +23,9 @@ Keys beyond the base contract:
 
 `--impl reference` times the reference's CPU algorithm (the oracle built for speed,
 oracle/liboracle_native.so, best thread count) on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes, after the timed steps, the consensus columns of the last step for a fixed, seeded
+sample of families (rank 0's shard), so that two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -38,17 +41,39 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # runs from the tree as build() left it, which may be read-only
 
 METRIC = "consensus reads/sec (simplex 150bp, depth-8 families)"
 UNIT = "consensus_reads/s"
 DEPTH, READ_LEN, ERR = 8, 150, 1e-3
 PARAMS = dict(error_rate_pre_umi=45, error_rate_post_umi=40, min_reads=1,
               min_consensus_base_quality=2)
+# --dump-outputs: 16384 families x 150 positions x 4 float32 columns = 39 MB
+DUMP_FAMILIES, DUMP_SEED = 16384, 20251017
 
 
 def algorithmic_bytes(n_units: int, n_reads: int, sum_len: int, sum_cons: int) -> int:
     """SURVEY §8(d): per unit 2*sum(len) in + 6*cons_len out + 8*(n_reads+1) + 8 index bytes."""
     return 2 * sum_len + 6 * sum_cons + 8 * (n_reads + n_units) + 8 * n_units
+
+
+def dump_outputs(torch, out_dir: str, host_batch, out, dev) -> None:
+    """Writes what fgb_vote_device left in `out` for a fixed, seeded sample of families: `base` (ASCII code),
+    `qual`, `depth` and `errors` as float32 [families, READ_LEN] arrays, and `family` (float64) the sampled
+    families' indices in the batch."""
+    n = host_batch.n_units
+    fams = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(DUMP_FAMILIES, n), replace=False))
+    units = host_batch.units
+    assert (units["cons_len"][fams] == READ_LEN).all()
+    pos = units["out_off"][fams].astype(np.int64)[:, None] + np.arange(READ_LEN, dtype=np.int64)[None, :]
+    idx = torch.from_numpy(pos).to(dev)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "family.npy"), fams.astype(np.float64))
+    for name, col in (("base", out.base), ("qual", out.qual), ("depth", out.depth), ("errors", out.errors)):
+        a = col[idx].cpu().numpy()
+        if a.dtype == np.int16:          # the device holds u16 counts in int16 tensors
+            a = a.view(np.uint16)
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
 
 
 def measured_peak_gbs():
@@ -402,9 +427,14 @@ def main():
     ap.add_argument("--record-families", type=int, default=int(os.environ.get("FGB_RECORD_FAMILIES", "200000")),
                     help="families per batch of the record-level leg")
     ap.add_argument("--no-modes", action="store_true", help="skip the duplex / CODEC / Zipf kernel legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's consensus columns for a seeded sample of "
+                         "families (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
+    if args.dump_outputs and args.impl != "fgumi_b200":
+        ap.error("--dump-outputs applies to --impl fgumi_b200")
 
     if args.impl == "reference":
         run_reference(args)                  # builds and loads oracle/ only: no product code on this arm
@@ -484,6 +514,8 @@ def main():
     total_ms = float(t.item())
     launches = eng.launch_count() - launches0
     stats_all = eng.stats()   # after the all-reduce every rank's block holds the global sums
+    if args.dump_outputs and rank == 0:
+        dump_outputs(torch, args.dump_outputs, tb.host, out, dev)
 
     value = U * world * args.steps / (total_ms * 1e-3)
     # ---- roofline of the dominant kernel (one launch per step) ----
